@@ -1,11 +1,14 @@
 #!/usr/bin/env python
-"""bench.py -- roko hot-path throughput on B200 (driver contract in the task brief).
+"""bench.py -- roko hot-path throughput on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 128]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 128] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* is one pass of the hot path (front end -> 3 x (projection, recurrence) -> head+argmax) over
-one batch of synthetic windows.  Workload at N=1: BASELINE.json configs[1] -- the 128-window batch of
+one batch of synthetic windows; the timed region is exactly K steps.  ``--dump-outputs DIR`` writes
+the labels of the last timed step (what ``RNN.predict`` returns to its caller) as ``DIR/labels.npy``
+(float32); the inputs are seeded, so two builds run with the same arguments can be compared output
+for output.  Workload at N=1: BASELINE.json configs[1] -- the 128-window batch of
 ``inference.py --b 128`` on synthetic (200 reads x 90 columns) uint8 windows with random-init weights
 (the reference-generated ``tests/golden/rand_seed1.pth``).  BASELINE.json's "200 pos x 30 reads" is
 not executable by the reference (SURVEY.md section 0.3); the geometry here is the reference's.
@@ -222,8 +225,9 @@ class StockTorchGpu:
         h, _ = self.gru(h.reshape(-1, 90, 500))                               # :56-57
         return torch.argmax(F.linear(h, sd["fc4.weight"], sd["fc4.bias"]), dim=2)   # :59, inference.py:116
 
-    def windows_per_s(self, pool, batch, min_s=0.4):
-        """Device-timed steady-state throughput at `batch` windows per call over a pool of resident inputs."""
+    def windows_per_s(self, pool, batch, steps=None, min_s=0.4):
+        """Device-timed steady-state throughput at `batch` windows per call over a pool of resident inputs:
+        exactly `steps` calls, or groups of 8 calls until `min_s` seconds when `steps` is None."""
         torch = self.torch
         xs = pool.view(-1, READS, COLS)
         n = xs.shape[0] // batch
@@ -233,14 +237,15 @@ class StockTorchGpu:
             torch.cuda.synchronize()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             done, ms = 0, 0.0
-            while ms < min_s * 1e3 and done < 2000:
+            while (done < steps) if steps else (ms < min_s * 1e3 and done < 2000):
+                k = min(8, steps - done) if steps else 8
                 e0.record()
-                for i in range(8):
+                for i in range(k):
                     self.predict(xs[((done + i) % n) * batch:((done + i) % n + 1) * batch])
                 e1.record()
                 torch.cuda.synchronize()
                 ms += e0.elapsed_time(e1)
-                done += 8
+                done += k
         return done * batch / (ms * 1e-3)
 
 
@@ -256,7 +261,7 @@ def run_torch_gpu(args):
     g = torch.Generator(device=dev).manual_seed(1234)
     pool = torch.randint(0, 12, (args.pool_batches, args.batch, READS, COLS), dtype=torch.uint8, device=dev, generator=g)
     stock = StockTorchGpu(sd, dev)
-    wps = stock.windows_per_s(pool, args.batch)
+    wps = stock.windows_per_s(pool, args.batch, steps=args.steps)
     print(json.dumps({
         "impl": "torch_gpu", "metric": "consensus_windows_per_sec", "value": wps, "unit": "windows/s", "n_gpus": 1,
         "steps": args.steps, "warmup": 3, "ms_per_step": args.batch / wps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -282,7 +287,7 @@ def run_ours(args):
     dev = torch.device("cuda", local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    batch, K, W, NS = args.batch, args.steps, max(3, args.warmup), args.streams
+    batch, K, W, NS = args.batch, args.steps, max(args.streams, args.warmup), args.streams
     peaks = load_peaks()
 
     # ---- model: rank 0 loads the .pth, NCCL-broadcasts the weights ---------------------------------
@@ -325,6 +330,7 @@ def run_ours(args):
     main = torch.cuda.current_stream(dev)
 
     def run_steps(n, out, src=None, first=0):
+        """n steps (one per 128-window batch, NS batches in flight) over pool batches first, first + 1, ..."""
         src = pool if src is None else src
         for s in streams:
             s.wait_stream(main)
@@ -334,45 +340,26 @@ def run_ours(args):
         for s in streams:
             main.wait_stream(s)
 
-    def block(first):
-        """K steps (one per 128-window batch, NS batches in flight) + this block's label gather when N > 1."""
-        run_steps(K, labels_all, first=first)
-        return rdist.gather_labels(labels_all.view(K * batch, COLS), K * batch * world) if world > 1 else None
-
+    sampler = ClockSampler(local_rank)
+    if rank == 0:
+        sampler.start()
+        time.sleep(0.12)
     with torch.no_grad():
+        # the warm-up gives every stream at least one step: its workspace and CUDA graph are made outside the timed region
         run_steps(W, labels_all)
+        if world > 1:
+            dist.barrier()
         torch.cuda.synchronize()
-        # The timed region is R blocks of exactly K steps, back to back (no sync between blocks).  R starts from a calibration
-        # block and is raised until the region lasts >= min_region seconds (the first blocks also pay the CUDA-graph captures).
-        block(0)
+        # the timed region is exactly K steps between one CUDA-event pair, plus their label gather when N > 1; they start
+        # at the pool batch after the warm-up's, so up to P - W steps read inputs no earlier step left in L2
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        tw0 = time.perf_counter()
+        e0.record(main)
+        run_steps(K, labels_all, first=W)
+        gathered = rdist.gather_labels(labels_all.view(K * batch, COLS), K * batch * world) if world > 1 else None
+        e1.record(main)
         torch.cuda.synchronize()
-        sampler = ClockSampler(local_rank)
-        if rank == 0:
-            sampler.start()
-            time.sleep(0.12)
-        R, regions = 8, []
-        for attempt in range(4):
-            if world > 1:
-                dist.barrier()
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            tw0 = time.perf_counter()
-            e0.record(main)
-            gathered = None
-            for r in range(R):
-                gathered = block(r * K)
-            e1.record(main)
-            torch.cuda.synchronize()
-            tw1 = time.perf_counter()
-            ms_try = e0.elapsed_time(e1)
-            if world > 1:                                # every rank takes the same decision
-                t = torch.tensor([ms_try], device=dev)
-                dist.all_reduce(t, op=dist.ReduceOp.MAX)
-                ms_try = float(t.item())
-            regions.append((tw0, tw1))
-            if ms_try >= args.min_region * 1e3 * 0.95 or R >= args.max_blocks:
-                break
-            R = min(args.max_blocks, int(np.ceil(R * args.min_region * 1e3 / max(ms_try, 1e-3) * 1.15)))
+        tw1 = time.perf_counter()
         if world > 1:
             dist.barrier()
         ms = e0.elapsed_time(e1)
@@ -380,10 +367,16 @@ def run_ours(args):
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
-    value = R * K * batch * world / (ms * 1e-3)
+    value = K * batch * world / (ms * 1e-3)
+
+    if args.dump_outputs and rank == 0:
+        # the last timed step's labels: this rank's batch, or every rank's batch in rank order as gathered on rank 0
+        last = gathered.view(world, K, batch, COLS)[:, K - 1].reshape(world * batch, COLS) if world > 1 else labels_all[K - 1]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "labels.npy"), last.cpu().numpy().astype(np.float32))
 
     # ---- N > 1: what rank 0 gathered over NVLink must equal, byte for byte, what ONE GPU computes for every
-    # rank's inputs (rank 0 regenerates each rank's seeded pool and replays that rank's last block) -----------
+    # rank's inputs (rank 0 regenerates each rank's seeded pool and replays that rank's timed steps) ----------
     shard_check = None
     if world > 1 and rank == 0:
         assert gathered is not None and gathered.shape == (K * batch * world, COLS)
@@ -392,7 +385,7 @@ def run_ours(args):
             for r in range(world):
                 src = pool if r == 0 else make_pool(r)
                 mine = torch.empty((K, batch, COLS), dtype=torch.uint8, device=dev)
-                run_steps(K, mine, src=src, first=(R - 1) * K)
+                run_steps(K, mine, src=src, first=W)
                 torch.cuda.synchronize()
                 ok = ok and bool(torch.equal(mine.view(K * batch, COLS), gathered[r * K * batch:(r + 1) * K * batch]))
                 del src
@@ -433,7 +426,7 @@ def run_ours(args):
         e2e_s = float(t.item())
     e2e_value = calls * Kh * batch * world / e2e_s
     # clocks sampled inside the two timed regions (device-resident steps, end-to-end calls)
-    clocks = sampler.stop([regions[-1], (t0, t0 + e2e_s)]) if rank == 0 else None
+    clocks = sampler.stop([(tw0, tw1), (t0, t0 + e2e_s)]) if rank == 0 else None
     del x_host
 
     # ---- per-kernel device times (CUDA events between the kernels of the chain) -> roofline --------
@@ -514,27 +507,26 @@ def run_ours(args):
     if rank == 0:
         line = {
             "metric": "consensus_windows_per_sec", "value": value, "unit": "windows/s", "n_gpus": world,
-            "steps": K, "warmup": W, "ms_per_step": ms / (R * K), "higher_is_better": True, "scaling": "weak",
+            "steps": K, "warmup": W, "ms_per_step": ms / K, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
-            "blocks": R, "timed_region_s": ms * 1e-3,
+            "timed_region_s": ms * 1e-3,
             "config": {
                 "workload": f"BASELINE configs[1]: batch={batch} synthetic windows (200 reads x 90 cols, uint8 codes 0..11) "
                             "per step on each GPU, random-init weights tests/golden/rand_seed1.pth, labels out (uint8)",
                 "batch": batch, "windows_per_step_all_gpus": batch * world, "parallelism": f"dp{world}",
                 "streams": NS,
-                "timing": f"{R} blocks of exactly {K} steps back to back between one CUDA-event pair (blocks repeat until the "
-                          f"region is >= {args.min_region} s so that a short --steps run is steady state); ms_per_step = region / ({R} x {K})",
+                "timing": f"exactly {K} steps between one CUDA-event pair after {W} warm-up steps; ms_per_step = region / {K}",
                 "e2e_note": "predict_host coalesces consecutive batches into device passes of <= 2368 windows "
                             "(windows are independent), so e2e can exceed the per-call batch-128 device number",
-                "l2": f"inputs cycle through a {P * batch * WIN_BYTES / 1e6:.0f} MB pool (> 126 MB L2)",
-                "collectives": ("ncclBroadcast weights %d B before timing; label all-gather of every block inside the timed region" % bcast_bytes)
+                "l2": f"step i reads batch ({W} + i) mod {P} of a {P * batch * WIN_BYTES / 1e6:.0f} MB pool (> 126 MB L2)",
+                "collectives": ("ncclBroadcast weights %d B before timing; label all-gather of the timed steps inside the timed region" % bcast_bytes)
                                if world > 1 else "none (1 GPU)",
                 "kernels": names,
             },
             "e2e": {"value": e2e_value, "unit": "windows/s", "h2d_bytes_per_step": batch * WIN_BYTES,
                     "d2h_bytes_per_step": batch * COLS, "api": "RNN.predict_host -> roko_b200_infer_host (pinned host buffers)",
                     "calls": calls, "windows_per_call": Kh * batch, "timed_region_s": e2e_s},
-            "gpu_launches": R * K * 8,
+            "gpu_launches": K * 8,
             "clocks": clocks,
             "parity": {"batch128_max_abs_logit_err": perr, "batch128_labels_exact": True,
                        "fixture": "tests/golden/golden_b128_seed1.npz (reference class outputs), same kernels as the timed loop",
@@ -637,7 +629,7 @@ def run_train(args):
     dev = torch.device("cuda", local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    K, W = min(args.steps, 200), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
@@ -664,7 +656,7 @@ def run_train(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--mode", default="infer", choices=["infer", "train"],
-                    help="infer: the north-star hot path (default, the driver's contract); train: the training step")
+                    help="infer: the north-star hot path (default); train: the training step")
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=1000)
     ap.add_argument("--warmup", type=int, default=10)
@@ -676,14 +668,19 @@ def main():
     ap.add_argument("--rec", type=int, default=None, help="tensor-core recurrence: 2 fp16 (default), 1 tf32")
     ap.add_argument("--front", type=int, default=None, help="front end: 0 mma.sync stages, 1 tcgen05 stages (library default if unset)")
     ap.add_argument("--graphs", type=int, default=None, help="CUDA-graph replay of the chain: 1 on (default), 0 off")
-    ap.add_argument("--min-region", type=float, default=0.5, help="repeat the K-step block until the timed region is this long (s)")
-    ap.add_argument("--max-blocks", type=int, default=2000)
+    ap.add_argument("--min-region", type=float, default=0.5, help="repeat the end-to-end predict_host call until its timed region is this long (s)")
     ap.add_argument("--no-library-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--pool-batches", type=int, default=64)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--coalesce", type=int, default=2368, help="windows in the coalesced device pass (extra fields)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the labels of the last timed step to DIR/labels.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs writes the outputs of the inference path (--impl ours --mode infer)")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "torch_gpu":
