@@ -86,6 +86,14 @@ int roko_b200_infer_host(roko_b200_model* m, const uint8_t* x_host, long long n_
  *   "front"         front end: 1 all contractions on tcgen05 (front_tc.cu, default), 0 SIMT gather + mma.sync (front.cu)
  *   "graphs"        replay the 8-kernel chain of roko_b200_forward_u8 as a CUDA graph (default 1; needs a non-default stream)
  *   "superbatch"    windows per device pass of roko_b200_infer_host (default 2368)
+ *   "geometry"      grids of the front end, the fp16-split projection and the head: 1 work-sized (default), 0 one CTA per unit of
+ *                   work up to the full chip (148 CTAs; the head 8 blocks per SM).  Geometry 1 gives each CTA at least
+ *                   "geo_front" windows (default 4), "geo_proj" 128x256 projection tiles (default 6) and "geo_head" rows
+ *                   (default 128), each 1 .. 1048576: a 128-window batch then runs on 32 / 45 / 90 CTAs instead of
+ *                   128 / 148 / 720, so each CTA spreads its fixed prologue over more work and, with several batches in
+ *                   flight on other streams, the SMs left free serve them (8.6 % more windows/s at 12 streams on a B200,
+ *                   for a longer single-batch latency, 0.88 instead of 0.67 ms; DESIGN.md section 4.1).  From 2368
+ *                   windows on both give the full chip.  Environment: ROKO_B200_GEOMETRY=0|1.  Training keeps full-chip grids.
  * The fp16-split kernels scale their operands by powers of two (weights x 256, activations x 16 / x 256); a GRU weight
  * with |w| >= 253 or a front-end activation >= 4062 (fc1 or fc2 output) leaves their range: roko_b200_model_check then returns
  * ROKO_B200_ERANGE and the tf32 kernels ("proj" 3, "rec" 1) serve such a model. */

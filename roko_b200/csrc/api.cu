@@ -75,8 +75,11 @@ int run_forward(roko_b200_model* m, const uint8_t* x, int n, float* logits, uint
     for (int c0 = 0; c0 < n; c0 += cap) {
         const int nc = (n - c0) < cap ? (n - c0) : cap;
         const int rows = nc * COLS;
+        const int front_ctas = launch_cap(m, nc, m->geo_front, m->num_sms);
+        const int proj_ctas = launch_cap(m, (long long)((rows + TC_BM - 1) / TC_BM) * (GI_N / TC_BN), m->geo_proj, m->num_sms);
+        const int head_ctas = launch_cap(m, rows, m->geo_head, HEAD_BLOCKS_PER_SM * m->num_sms);
         if (ev) CU(cudaEventRecord(ev[0], s));
-        if (m->front_kind == 1) CU(launch_front_tc(x + (size_t)c0 * WIN_BYTES, pk, u, nc, m->status, m->num_sms, s));
+        if (m->front_kind == 1) CU(launch_front_tc(x + (size_t)c0 * WIN_BYTES, pk, u, nc, m->status, front_ctas, s));
         else CU(launch_front(x + (size_t)c0 * WIN_BYTES, pk, u, nc, m->status, m->num_sms, s));
         if (taps && taps->front)
             CU(cudaMemcpy2DAsync(taps->front, IN0 * sizeof(float), u, IN0P * sizeof(float), IN0 * sizeof(float),
@@ -85,7 +88,7 @@ int run_forward(roko_b200_model* m, const uint8_t* x, int n, float* logits, uint
         float* outs[3] = {h0, h1, h0};
         for (int l = 0; l < LAYERS; ++l) {
             if (ev) CU(cudaEventRecord(ev[1 + 2 * l], s));
-            CU(proj_dispatch(m, in, l, gi, rows, s));
+            CU(proj_dispatch(m, in, l, gi, rows, proj_ctas, s));
             if (ev) CU(cudaEventRecord(ev[2 + 2 * l], s));
             CU(rec_dispatch(m, gi, l, outs[l], nc, s));
             if (taps && taps->gru[l])
@@ -95,7 +98,7 @@ int run_forward(roko_b200_model* m, const uint8_t* x, int n, float* logits, uint
         }
         if (ev) CU(cudaEventRecord(ev[7], s));
         CU(launch_head(in, pk + PK_W4, pk + PK_B4, logits ? logits + (size_t)c0 * COLS * CLASSES : nullptr,
-                       labels ? labels + (size_t)c0 * COLS : nullptr, rows, s));
+                       labels ? labels + (size_t)c0 * COLS : nullptr, rows, head_ctas, s));
         if (ev) CU(cudaEventRecord(ev[8], s));
     }
     return ROKO_B200_OK;
@@ -265,6 +268,7 @@ int roko_b200_model_create(roko_b200_model** out, int device) {
     if (const char* rk = getenv("ROKO_B200_REC")) m->rec_kind = strcmp(rk, "tf32") == 0 ? 1 : 2;
     if (const char* gr = getenv("ROKO_B200_GRAPHS")) m->use_graphs = atoi(gr);
     if (const char* fr = getenv("ROKO_B200_FRONT")) m->front_kind = strcmp(fr, "tc") == 0 ? 1 : 0;
+    if (const char* ge = getenv("ROKO_B200_GEOMETRY")) m->geometry = atoi(ge) != 0;
     if (e != cudaSuccess) {
         roko_b200_model_destroy(m);
         return fail(ROKO_B200_ECUDA, "model_create: %s%s", cudaGetErrorString(e));
@@ -439,6 +443,10 @@ int roko_b200_model_set_option(roko_b200_model* m, const char* name, long long v
     if (strcmp(name, "rec") == 0) { if (value != 1 && value != 2) return fail(ROKO_B200_EARG, "rec must be 1 (tf32) or 2 (fp16)%s%s"); m->rec_kind = (int)value; return ROKO_B200_OK; }
     if (strcmp(name, "graphs") == 0) { m->use_graphs = value != 0; return ROKO_B200_OK; }
     if (strcmp(name, "front") == 0) { if (value != 0 && value != 1) return fail(ROKO_B200_EARG, "front must be 0 (mma.sync) or 1 (tcgen05)%s%s"); m->front_kind = (int)value; return ROKO_B200_OK; }
+    if (strcmp(name, "geometry") == 0) { if (value != 0 && value != 1) return fail(ROKO_B200_EARG, "geometry must be 0 (full-chip grids) or 1 (work-sized grids)%s%s"); m->geometry = (int)value; return ROKO_B200_OK; }
+    int* geo = strcmp(name, "geo_front") == 0 ? &m->geo_front : strcmp(name, "geo_proj") == 0 ? &m->geo_proj
+             : strcmp(name, "geo_head") == 0 ? &m->geo_head : nullptr;
+    if (geo) { if (value < 1 || value > (1 << 20)) return fail(ROKO_B200_EARG, "%s must be 1 .. 1048576%s", name); *geo = (int)value; return ROKO_B200_OK; }
     return fail(ROKO_B200_EARG, "unknown option '%s'%s", name);
 }
 

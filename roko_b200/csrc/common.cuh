@@ -143,8 +143,9 @@ cudaError_t launch_proj_tc3(const float* A, int K, const float* wimg, const floa
                             int num_sms, cudaStream_t s);
 cudaError_t proj_tc3_setup();
 // fp16-split projection (proj_h.cu): in_scale = power-of-two scale applied to A before the split (tc::U_SCALE / tc::H_SCALE)
+// max_ctas caps the grid (at most one CTA per 128x256 tile); the CTAs stride over the tiles, so it moves no arithmetic
 cudaError_t launch_proj_h(const float* A, int K, const float* wimg, const float* bias, float* C, int M, float in_scale,
-                          int* status, int num_sms, cudaStream_t s);
+                          int* status, int max_ctas, cudaStream_t s);
 cudaError_t proj_h_setup();
 // fp16-split recurrence (rec_h.cu): rh16_d0 = pk_rh16(l, 0), directions RH16_DIR floats apart
 cudaError_t launch_rec_h(const float* gi, const float* rh16_d0, float* out, int nwin, int num_sms, cudaStream_t s);
@@ -154,11 +155,14 @@ cudaError_t launch_rec_tc(const float* gi, const float* whi_d0, const float* wlo
 cudaError_t rec_tc_setup();
 cudaError_t launch_rec(const float* gi, const float* whh_d0, size_t dir_stride, const float* bhn_d0,
                        float* out, int nwin, int num_sms, cudaStream_t s);
+// head (head.cu): at most max_blocks blocks of 8 warps, two rows per warp and pass; HEAD_BLOCKS_PER_SM x SMs is the full chip
+constexpr int HEAD_BLOCKS_PER_SM = 8;
 cudaError_t launch_head(const float* h, const float* w4, const float* b4, float* logits, uint8_t* labels,
-                        int rows, cudaStream_t s);
+                        int rows, int max_blocks, cudaStream_t s);
 cudaError_t measure_fp32_peak(double* tflops);
 cudaError_t front_setup();
-cudaError_t launch_front_tc(const uint8_t* x, const float* packed, float* u, int nwin, int* status, int num_sms,
+// front_tc.cu: at most max_ctas persistent CTAs (one per SM), each walking windows blockIdx.x, blockIdx.x + gridDim.x, ...
+cudaError_t launch_front_tc(const uint8_t* x, const float* packed, float* u, int nwin, int* status, int max_ctas,
                             cudaStream_t s);
 cudaError_t front_tc_setup();
 cudaError_t rec_setup();

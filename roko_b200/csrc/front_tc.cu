@@ -451,10 +451,11 @@ cudaError_t front_tc_setup() {
     return cudaFuncSetAttribute(front_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FT_SMEM);
 }
 
-cudaError_t launch_front_tc(const uint8_t* x, const float* packed, float* u, int nwin, int* status, int num_sms,
+cudaError_t launch_front_tc(const uint8_t* x, const float* packed, float* u, int nwin, int* status, int max_ctas,
                             cudaStream_t s) {
     if (nwin <= 0) return cudaSuccess;
-    const int grid = nwin < num_sms ? nwin : num_sms;
+    if (max_ctas < 1) return cudaErrorInvalidValue;
+    const int grid = nwin < max_ctas ? nwin : max_ctas;
     front_tc_kernel<<<grid, FT_THREADS, FT_SMEM, s>>>(x, packed, u, nwin, status);
     return cudaGetLastError();
 }

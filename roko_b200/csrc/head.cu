@@ -66,10 +66,11 @@ head_kernel(const float* __restrict__ h, const float* __restrict__ w4, const flo
 }
 
 cudaError_t launch_head(const float* h, const float* w4, const float* b4, float* logits, uint8_t* labels,
-                        int rows, cudaStream_t s) {
+                        int rows, int max_blocks, cudaStream_t s) {
     if (rows <= 0) return cudaSuccess;
+    if (max_blocks < 1) return cudaErrorInvalidValue;
     int blocks = ((rows + 1) / 2 + (HD_THREADS / 32) - 1) / (HD_THREADS / 32);
-    if (blocks > 148 * 8) blocks = 148 * 8;
+    if (blocks > max_blocks) blocks = max_blocks;
     head_kernel<<<blocks, HD_THREADS, 0, s>>>(h, w4, b4, logits, labels, rows);
     return cudaGetLastError();
 }

@@ -8,6 +8,8 @@
 #include "tc.cuh"
 
 constexpr int NSLOT = 3;
+// launch geometry of the inference chain (launch_cap): least work per CTA of front_tc (windows), proj_h (128x256 tiles) and head (rows)
+constexpr int GEO_FRONT_DEFAULT = 4, GEO_PROJ_DEFAULT = 6, GEO_HEAD_DEFAULT = 128;
 constexpr int ROKO_ERRBUF = 512;
 char* roko_b200_errbuf();         // the calling thread's roko_b200_last_error() buffer (api.cu)
 
@@ -63,6 +65,11 @@ struct roko_b200_model {
     int use_graphs = 1;             // replay the chain as a CUDA graph when the batch fits the workspace (ROKO_B200_GRAPHS=0 disables)
     int front_kind = 1;             // front end: 1 = all three contractions on tcgen05 (front_tc.cu, default); 0 = SIMT gather + warp-level
                                     // mma.sync stages (front.cu, round 1).  ROKO_B200_FRONT=tc|mma
+    int geometry = 1;               // grids of front_tc / proj_h / head in the inference chain (launch_cap): 1 = at least geo_* units of
+                                    // work per CTA, 0 = one CTA per unit up to the full chip.  ROKO_B200_GEOMETRY=0|1
+    int geo_front = GEO_FRONT_DEFAULT;  // windows per front_tc CTA at least
+    int geo_proj = GEO_PROJ_DEFAULT;    // 128x256 tiles per proj_h CTA at least
+    int geo_head = GEO_HEAD_DEFAULT;    // rows per head block at least
 };
 
 // offset of raw element `off` inside raw_al (RAW_GRU is 2 mod 4 and every later tensor size is a multiple of 4)
@@ -70,14 +77,26 @@ constexpr int RAW_AL_PAD = 2;
 static_assert((roko::RAW_GRU + RAW_AL_PAD) % 4 == 0 && roko::RAW_W1 % 4 == 0 && roko::RAW_W2 % 4 == 0, "raw_al alignment");
 __host__ __device__ constexpr int raw_al_off(int off) { return off >= roko::RAW_GRU ? off + RAW_AL_PAD : off; }
 
-// Input projection of GRU layer `l` with the kernel the model is configured for (see use_tc).
-inline cudaError_t proj_dispatch(const roko_b200_model* m, const float* in, int l, float* gi, int rows,
+// Grid of a launch over `units` of work with CTA limit `full`.  Geometry 1 gives each CTA at least `min_per_cta` units: every
+// CTA pays its prologue (tensor-memory images, barrier set-up, pipeline fill and drain) once per launch, so a 128-window batch
+// on 148 CTAs spends a large share of its SM-time there, while with several batches in flight on other streams the SMs a smaller grid
+// leaves free run their kernels.  Batches large enough for `full` CTAs at `min_per_cta` get `full` either way.  The kernels
+// stride their work by gridDim.x, so the grid changes no result.
+inline int launch_cap(const roko_b200_model* m, long long units, int min_per_cta, int full) {
+    if (!m->geometry) return full;
+    const long long ctas = (units + min_per_cta - 1) / min_per_cta;
+    return ctas < 1 ? 1 : (ctas < full ? (int)ctas : full);
+}
+
+// Input projection of GRU layer `l` with the kernel the model is configured for (see use_tc); proj_ctas caps the grid of the
+// fp16-split kernel (the tf32 and FFMA kernels keep their own).
+inline cudaError_t proj_dispatch(const roko_b200_model* m, const float* in, int l, float* gi, int rows, int proj_ctas,
                                  cudaStream_t s) {
     using namespace roko;
     const float* pk = m->packed;
     if (m->use_tc == 4)
         return launch_proj_h(in, gru_inp(l), pk + pk_wh16(l), pk + pk_bgi(l), gi, rows, l == 0 ? tc::U_SCALE : tc::H_SCALE,
-                             m->status, m->num_sms, s);
+                             m->status, proj_ctas, s);
     if (m->use_tc == 3) return launch_proj_tc3(in, gru_inp(l), pk + pk_wtc(l), pk + pk_bgi(l), gi, rows, m->num_sms, s);
     return launch_proj(in, gru_inp(l), pk + pk_wih(l), pk + pk_bgi(l), gi, rows, s);
 }

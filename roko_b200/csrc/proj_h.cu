@@ -251,10 +251,11 @@ cudaError_t proj_h_setup() {
 }
 
 cudaError_t launch_proj_h(const float* A, int K, const float* wimg, const float* bias, float* C, int M, float in_scale,
-                          int* status, int num_sms, cudaStream_t s) {
+                          int* status, int max_ctas, cudaStream_t s) {
     if (M <= 0) return cudaSuccess;
+    if (max_ctas < 1) return cudaErrorInvalidValue;
     const int ntiles = ((M + TC_BM - 1) / TC_BM) * (GI_N / TC_BN);
-    const int grid = ntiles < num_sms ? ntiles : num_sms;
+    const int grid = ntiles < max_ctas ? ntiles : max_ctas;
     if (K == IN0P) proj_h_kernel<IN0P><<<grid, PH_THREADS, PH_SMEM, s>>>(A, wimg, bias, C, M, ntiles, in_scale, status);
     else if (K == OUT_W) proj_h_kernel<OUT_W><<<grid, PH_THREADS, PH_SMEM, s>>>(A, wimg, bias, C, M, ntiles, in_scale, status);
     else return cudaErrorInvalidValue;

@@ -132,7 +132,7 @@ int roko_b200_train_forward(roko_b200_model* m, const uint8_t* x, int n_windows,
     const float* in = w.u;
     const size_t dstride = (size_t)(pk_whh(0, 1) - pk_whh(0, 0));
     for (int l = 0; l < LAYERS; ++l) {
-        TCU(proj_dispatch(m, in, l, w.gi, rows, s));
+        TCU(proj_dispatch(m, in, l, w.gi, rows, m->num_sms, s));       // one stream: the whole chip
         TCU(launch_rec_train(w.gi, pk + pk_whh(l, 0), dstride, pk + pk_bhn(l, 0), w.out[l],
                              reinterpret_cast<float4*>(w.gates[l]), n_windows, m->num_sms, s));
         if (l + 1 < LAYERS) {                                                   // nn.GRU(dropout=...): between layers only
@@ -140,7 +140,7 @@ int roko_b200_train_forward(roko_b200_model* m, const uint8_t* x, int n_windows,
             in = w.outd[l];
         }
     }
-    TCU(launch_head(w.out[LAYERS - 1], pk + PK_W4, pk + PK_B4, logits, nullptr, rows, s));
+    TCU(launch_head(w.out[LAYERS - 1], pk + PK_W4, pk + PK_B4, logits, nullptr, rows, HEAD_BLOCKS_PER_SM * m->num_sms, s));
     return ROKO_B200_OK;
 }
 

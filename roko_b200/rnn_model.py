@@ -349,7 +349,8 @@ class RNN(nn.Module):
 
     def set_option(self, name, value, device=None):
         """Scheduling / kernel-selection knobs of the C library (see include/roko_b200.h): rec_tc_min, superbatch,
-        proj (0 ffma, 3 tf32, 4 fp16), rec (1 tf32, 2 fp16), front (0 mma.sync, 1 tcgen05), graphs (0/1)."""
+        proj (0 ffma, 3 tf32, 4 fp16), rec (1 tf32, 2 fp16), front (0 mma.sync, 1 tcgen05), graphs (0/1), geometry (0 full-chip,
+        1 work-sized grids) and its minima geo_front / geo_proj / geo_head."""
         dev = torch.device(device) if device is not None else next(self.parameters()).device
         h = self._handle(dev)
         _cabi.check(h.lib.roko_b200_model_set_option(h.ptr, name.encode(), int(value)))
